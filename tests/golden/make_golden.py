@@ -14,12 +14,18 @@ Fixtures:
   *.fna.gz                      the two real genomes of the reference's tests/data (gzip -9)
   tricky.fq + tricky.contigs.txt  a hand-made FASTA/FASTQ mix and what the reference's kseq_read yields for it
                                 (name, length, crc32 per record; `ref_dump contigs`)
+  synth_ref.json                `make_golden.py synthetic` only: the seeded genome set of tests/test_oracle.py
+                                (synthetic_set) through `ref_dump map` (row count + SHA-256, query fragment total per
+                                query) and through fastANI_ref (output lines, FASTA directory stripped)
 """
 import hashlib
 import json
 import os
+import re
+import shutil
 import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -122,5 +128,37 @@ def main():
     print("golden fixtures written to", HERE)
 
 
+def synthetic():
+    sys.path[:0] = [ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")]
+    from test_oracle import SYNTH_QUERIES, synthetic_set
+    tmp = tempfile.mkdtemp()
+    paths = []
+    for g, contigs in enumerate(synthetic_set()):
+        paths.append(os.path.join(tmp, "g%d.fa" % g))
+        with open(paths[-1], "wb") as f:
+            for name, seq in contigs:
+                f.write(b">" + name.encode() + b" synthetic\n")
+                for o in range(0, len(seq), 70):
+                    f.write(seq[o:o + 70] + b"\n")
+    ql, rl, out_txt, out_map = (os.path.join(tmp, n) for n in ("ql.txt", "rl.txt", "out.txt", "q.map"))
+    open(ql, "w").write("\n".join(paths[i] for i in SYNTH_QUERIES) + "\n")
+    open(rl, "w").write("\n".join(paths) + "\n")
+    golden = {}
+    for k, L in ((16, 3000), (16, 1000), (21, 5000)):
+        case = {}
+        for qi in SYNTH_QUERIES:
+            r = run(DUMP, "map", str(k), str(L), out_map, paths[qi], *paths)
+            b = open(out_map, "rb").read()
+            case["q%d" % qi] = {"records": len(b) // 44, "sha256": hashlib.sha256(b).hexdigest(),
+                                "total_fragments": int(re.search(r"totalQueryFragments=(\d+)", r.stderr).group(1))}
+        run(CLI, "--ql", ql, "--rl", rl, "-k", str(k), "--fragLen", str(L), "-t", "2", "-o", out_txt)
+        case["out_txt"] = ["\t".join(os.path.basename(f) if f.startswith(tmp) else f for f in ln.split("\t"))
+                           for ln in open(out_txt).read().splitlines()]
+        golden["k%d.L%d" % (k, L)] = case
+    shutil.rmtree(tmp)
+    json.dump(golden, open(os.path.join(HERE, "synth_ref.json"), "w"), indent=1)
+    print("synth_ref.json written to", HERE)
+
+
 if __name__ == "__main__":
-    sys.exit(main())
+    sys.exit(synthetic() if sys.argv[1:] == ["synthetic"] else main())

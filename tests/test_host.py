@@ -209,6 +209,28 @@ def test_bench_parity_gate_detects_every_kind_of_difference():
     assert cfg["queries"] == 1000 and "4 GPU" in cfg["parallelism"]
 
 
+def test_bench_output_dump(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: the dense tables as float arrays, exact; above the byte budget the same seeded sample of
+    query rows every time, listed in query_index.npy, and the files stay within the budget."""
+    import bench
+    rng = np.random.default_rng(1)
+    cnt = rng.integers(0, 1667, (300, 40)).astype(np.int32)
+    idn = rng.uniform(80, 100, (300, 40)).astype(np.float32)
+    tot = rng.integers(1, 1667, 300).astype(np.int32)
+    bench.dump_outputs(str(tmp_path / "all"), cnt, idn, tot)
+    ld = lambda d, n: np.load(str(tmp_path / d / (n + ".npy")))
+    assert ld("all", "count_seq").dtype == np.float64 and (ld("all", "count_seq") == cnt).all()
+    assert ld("all", "identity").dtype == np.float32 and (ld("all", "identity").view(np.uint32) == idn.view(np.uint32)).all()
+    assert (ld("all", "total_query_fragments") == tot).all() and not (tmp_path / "all" / "query_index.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_BUDGET", 20000)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), cnt, idn, tot)
+    q = ld("s1", "query_index").astype(np.int64)
+    assert 0 < len(q) < 300 and (np.diff(q) > 0).all() and (q == ld("s2", "query_index")).all()
+    assert (ld("s1", "count_seq") == cnt[q]).all() and (ld("s1", "total_query_fragments") == tot[q]).all()
+    assert sum(os.path.getsize(tmp_path / "s1" / f) - 128 for f in os.listdir(tmp_path / "s1")) <= 20000     # 128 B .npy headers
+
+
 def test_host_packer_matches_the_reference_bytes():
     """bani_pack_contig (no GPU): decoding the 2-bit words and patching the exception list gives back exactly the
     upper-cased bytes the reference hashes (makeUpperCase touches a-z only, commonFunc.hpp:57-66)."""

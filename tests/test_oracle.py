@@ -137,31 +137,18 @@ def test_degenerate_k21_L1000(genomes):
     assert json.load(open(os.path.join(GOLDEN, "sweep.json")))["21,1000"] == ""
 
 
-def _write_fasta(path, contigs, width=70):
-    with open(path, "wb") as f:
-        for name, seq in contigs:
-            f.write(b">" + name.encode() + b" synthetic\n")
-            for o in range(0, len(seq), width):
-                f.write(seq[o:o + width] + b"\n")
+SYNTH_QUERIES = (0, 1, 3)
 
 
-@pytest.mark.parametrize("k,L", [(16, 3000), (16, 1000), (21, 5000)])
-def test_oracle_against_the_compiled_reference_on_fresh_synthetic_genomes(tmp_path, k, L):
-    """Beyond the committed fixtures: the C restatement against oracle/_ref (the UNMODIFIED reference compiled by
-    oracle/Makefile) run live on a seeded multi-contig set with N runs, lower case, short contigs and repeats --
-    every MappingResult row byte for byte, and the CLI's output lines."""
-    import subprocess
-    from conftest import ROOT
+def synthetic_set():
+    """Four seeded 60 kbp genomes: one multi-contig genome with lower case, an N run, a contig shorter than a fragment
+    and a tandem repeat; one cut in two; two in one piece."""
     from fastani_b200.synth import synth_genome
-    dump = os.path.join(ROOT, "oracle", "_ref", "ref_dump")
-    cli = os.path.join(ROOT, "oracle", "_ref", "fastANI_ref")
-    if not (os.path.exists(dump) and os.path.exists(cli)):
-        pytest.skip("oracle/_ref has not been built (needs /root/reference)")
     Lg = 60000
     genomes = []
     for g in range(4):
         a = synth_genome(21, 1 + g // 3, g % 3, 25000 * (g % 3), Lg).tobytes()
-        if g == 1:      # multi-contig, lower case, an N run, a contig shorter than a fragment, a tandem repeat
+        if g == 1:
             contigs = [("g1_a", a[:21000].lower()), ("g1_tiny", a[21000:21500]), ("g1_b", a[21500:40000] + b"N" * 333 + a[40000:52000]),
                        ("g1_rep", (a[52000:52060] * 60)), ("g1_c", a[52060:])]
         elif g == 2:
@@ -169,32 +156,28 @@ def test_oracle_against_the_compiled_reference_on_fresh_synthetic_genomes(tmp_pa
         else:
             contigs = [("g%d" % g, a)]
         genomes.append(contigs)
-    paths = []
-    for g, contigs in enumerate(genomes):
-        p = str(tmp_path / ("g%d.fa" % g))
-        _write_fasta(p, contigs)
-        paths.append(p)
+    return genomes
+
+
+@pytest.mark.parametrize("k,L", [(16, 3000), (16, 1000), (21, 5000)])
+def test_oracle_against_the_compiled_reference_on_fresh_synthetic_genomes(k, L):
+    """Beyond the real-genome fixtures: the C restatement against what the UNMODIFIED reference (oracle/_ref, compiled by
+    oracle/Makefile) computed for synthetic_set() written as g0.fa ... g3.fa (tests/golden/synth_ref.json, written by
+    `make_golden.py synthetic`) -- every MappingResult row byte for byte (as a SHA-256), the query fragment totals, and
+    the CLI's output lines."""
+    genomes = synthetic_set()
+    names = ["g%d.fa" % g for g in range(len(genomes))]
+    want = json.load(open(os.path.join(GOLDEN, "synth_ref.json")))["k%d.L%d" % (k, L)]
     w = po.lib().orc_window_size(k, L)
     rec, sbf, _ = po.sketch_genomes(genomes, k, w)
     ix = po.Index(rec)
     results, qlens = [], [genome_length([len(s) for _, s in g], L) for g in genomes]
-    for qi in (0, 1, 3):
-        out = str(tmp_path / ("q%d.map" % qi))
-        r = subprocess.run([dump, "map", str(k), str(L), out, paths[qi]] + paths, capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr
-        want = open(out, "rb").read()
+    for j, qi in enumerate(SYNTH_QUERIES):
         rows, tot, _ = po.map_genome(ix, genomes[qi], k, w, L)
-        assert rows.tobytes() == want, (qi, len(rows), len(want) // 44)
-        assert ("totalQueryFragments=%d" % tot) in r.stderr
-        results += [([0, 1, 3].index(qi), gid, c, tot, idn) for gid, c, idn in po.cgi(rows, sbf, L)]
+        ref = want["q%d" % qi]
+        assert len(rows) == ref["records"] and hashlib.sha256(rows.tobytes()).hexdigest() == ref["sha256"], (qi, len(rows), ref["records"])
+        assert tot == ref["total_fragments"]
+        results += [(j, gid, c, tot, idn) for gid, c, idn in po.cgi(rows, sbf, L)]
     assert len(results) >= 4
-    # the reference CLI on the same files
-    ql, rl = str(tmp_path / "ql.txt"), str(tmp_path / "rl.txt")
-    open(ql, "w").write("\n".join(paths[i] for i in (0, 1, 3)) + "\n")
-    open(rl, "w").write("\n".join(paths) + "\n")
-    r = subprocess.run([cli, "--ql", ql, "--rl", rl, "-k", str(k), "--fragLen", str(L), "-t", "2", "-o", str(tmp_path / "out.txt")],
-                       capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr[-1000:]
-    got = open(tmp_path / "out.txt").read().splitlines()
-    want = output_lines(results, [paths[i] for i in (0, 1, 3)], paths, [qlens[i] for i in (0, 1, 3)], qlens, L, 0.2)
-    assert sorted(got) == sorted(want)
+    got = output_lines(results, [names[i] for i in SYNTH_QUERIES], names, [qlens[i] for i in SYNTH_QUERIES], qlens, L, 0.2)
+    assert sorted(got) == sorted(want["out_txt"])
